@@ -9,6 +9,7 @@ independent streams, no collective on the data path).  One "step" = one block of
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [...]                         # the reference's CPU path
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+    python bench.py --dump-outputs DIR [...]                       # also write the timed paths' last outputs
 
 Prints ONE JSON line on rank 0.
   value         device-resident throughput (inputs in HBM).  The timed region is closed over EVERY stream the
@@ -21,6 +22,12 @@ Prints ONE JSON line on rank 0.
   cpu_baseline  the compiled reference (oracle/_ref) on this box's host cores over a bounded sample.
   configs       (1 GPU runs) driver-run numbers for BASELINE configs 2-5, the CLI-default 2048-frame block, and
                 `e2e_dropin`: run_effects_chain() of the reference's chain runtime with the GPU effects linked in.
+
+With --dump-outputs DIR, rank 0 also writes the block the headline and e2e paths returned in their last timed step
+as DIR/<name>.npy (float64, [frames, channels]; at most 64 MB = 64e6 bytes in all, beyond that a fixed, seeded sample
+of frames): `device` (the headline's device-resident call), `host` and `host_pipelined` (the two host-call legs of
+`e2e`, unless --no-e2e).  The configs are not dumped.  Inputs and IRs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import math
@@ -73,6 +80,24 @@ def make_irs(taps, channels, first_channel=0):
 def make_block(frames, channels, seed):
     u = park_miller(1000 + seed, frames * channels) / 2147483647.0 - 0.5
     return u.reshape(frames, channels)
+
+
+DUMP_LIMIT = 64 * 10 ** 6          # bytes of all files together, .npy headers included
+NPY_HEADER_MAX = 4096
+
+
+def dump_outputs(path, arrays):
+    """arrays: name -> [frames, channels].  Each goes to path/<name>.npy as float64; when the files would exceed
+    DUMP_LIMIT bytes together, every array is cut to the same fixed, seeded sample of its frames (sorted)."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    budget = DUMP_LIMIT - NPY_HEADER_MAX * len(arrays)
+    for name, v in arrays.items():
+        if total > budget:
+            keep = max(1, v.shape[0] * budget // total)
+            v = v[np.sort(np.random.default_rng(0).choice(v.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), v)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -492,6 +517,7 @@ def main():
     ap.add_argument("--no-kernels", action="store_true", help="skip the per-kernel (serialised) timing pass")
     ap.add_argument("--e2e-slabs", type=int, default=4, help="channel slabs of the synchronous host call (copy-in / kernels / copy-out of the slabs overlap)")
     ap.add_argument("--e2e-pipe-slabs", type=int, default=0, help="channel slabs with blocks in flight (0: same as --e2e-slabs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output of the headline and e2e paths as DIR/<name>.npy (device, host, host_pipelined)")
     a = ap.parse_args()
 
     # stdout carries exactly one JSON line: whatever libraries print there (NCCL's version banner under
@@ -561,6 +587,7 @@ def main():
     total_samples = float(world) * C * F * steps
     value = total_samples / (ms * 1e-3) / 1e6
     checksum = float(d_out.abs().sum().item())
+    outputs = {"device": d_out.cpu().numpy()} if a.dump_outputs else {}     # before the per-kernel pass reuses d_out
 
     plan = [op for op in chain.describe() if op.get("op") == "fir"][0]
     h = 0 if a.shared_ir else 1
@@ -649,6 +676,8 @@ def main():
         e2e = {"value": total_samples / dt / 1e6, "unit": UNIT, "h2d_bytes_per_step": F * C * 8, "d2h_bytes_per_step": F * C * 8,
                "ms_per_step": dt / steps * 1e3, "api": "dspb200_chain_run_host, pinned host buffers (inputs write-combined), %d channel slabs" % a.e2e_slabs,
                "numa": numa, "checksum": float(np.abs(pout.array).sum())}
+        if a.dump_outputs:
+            outputs["host"] = pout.array.copy()
         # the same blocks through submit/wait: up to `depth` blocks in flight, each with its own output buffer
         depth = 3
         pslabs = a.e2e_pipe_slabs or a.e2e_slabs
@@ -679,10 +708,14 @@ def main():
                             "host_submit_ms_per_step": t_submit / steps * 1e3, "blocks_in_flight": depth, "channel_slabs": pslabs,
                             "api": "dspb200_chain_submit_host + dspb200_chain_wait (same copies, same kernels; the synchronous call above is what the drop-in effect->run() uses)",
                             "checksum": float(np.abs(pouts[(steps - 1) % (depth + 1)].array).sum())}
+        if a.dump_outputs:
+            outputs["host_pipelined"] = pouts[(steps - 1) % (depth + 1)].array.copy()
         ch2.close()
 
     clocks = sampler.stop()          # sampled across both timed loops (device-resident and host-call)
     launches_total = int(reduce_sum(float(launches)))
+    if outputs and rank == 0:
+        dump_outputs(a.dump_outputs, outputs)
 
     configs = None
     if rank == 0 and world == 1 and not a.no_configs:

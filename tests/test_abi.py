@@ -51,25 +51,16 @@ def test_product_never_imports_oracle():
                     assert not pat.search(text), "%s reaches into the oracle" % os.path.join(dirpath, f)
 
 
-def test_host_side_design_matches_reference(have_ref):
-    """biquad.c:111-294 coefficient design, bit for bit (host arithmetic, no GPU needed)."""
-    if not have_ref:
-        pytest.skip("compiled reference not available")
+def test_host_side_design_matches_reference():
+    """biquad.c:111-294 coefficient design, bit for bit (host arithmetic, no GPU needed), against the compiled
+    reference's designs of every type and width type (tests/golden/ref_biquad_design.npz, make_golden.py)."""
     import numpy as np
     import dsp_b200
-    from oracle import ref
-    for t in range(1, 16):
-        for wt in (1, 2, 3, 4, 5):
-            if wt in (2, 3) and t not in (14, 15):
-                continue
-            for f0, w, g in [(1000, 0.7, 3.0), (31.25, 1.4, -2), (16000, 0.5, 6), (100, 2.0, -9.5)]:
-                a = dsp_b200.biquad_design(t, 48000, f0, w, g, 0, wt)
-                b = ref.biquad_design(t, 48000, f0, w, g, 0, wt)
-                assert np.array_equal(a, b), (t, wt, f0, a, b)
-    for t in (16, 17):
-        a = dsp_b200.biquad_design(t, 44100, 50, 0.7, 20, 0.5, 1)
-        b = ref.biquad_design(t, 44100, 50, 0.7, 20, 0.5, 1)
-        assert np.array_equal(a, b)
+    g = np.load(os.path.join(ROOT, "tests", "golden", "ref_biquad_design.npz"))
+    assert len(g["args"]) == 15 * 3 * 4 + 2 * 2 * 4 + 2
+    for (t, fs, f0, w, gain, a3, wt), b in zip(g["args"], g["coefs"]):
+        a = dsp_b200.biquad_design(int(t), fs, f0, w, gain, a3, int(wt))
+        assert np.array_equal(a, b), (t, wt, f0, a, b)
 
 
 def test_helpers_match_restatement():

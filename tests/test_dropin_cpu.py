@@ -31,7 +31,7 @@ def test_shim_exports_reference_symbols():
     """The replacement objects export exactly the symbols the reference's biquad.o fir.o fir_p.o hilbert.o
     resample.o export (SURVEY.md 8b)."""
     import subprocess
-    objdir = os.path.join(os.path.dirname(HERE), "shim", "_build", "obj")
+    objdir = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "dropin", "shim")
     if not os.path.isdir(objdir):
         pytest.skip("shim objects not built")
     want = {"biquad.o": {"biquad_effect_init", "biquad_init", "biquad_reset", "biquad_init_using_type"},
@@ -50,7 +50,7 @@ def test_align_entry_point_and_fallback_symbols():
     ref_align_effect_insert (renamed with objcopy) as the host implementation for chains without GPU effects."""
     import subprocess
     root = os.path.dirname(HERE)
-    obj, ref = os.path.join(root, "shim", "_build", "obj", "align.o"), os.path.join(root, "shim", "_build", "ref", "align.o")
+    obj, ref = os.path.join(root, "oracle", "_ref", "dropin", "shim", "align.o"), os.path.join(root, "oracle", "_ref", "dropin", "ref", "align.o")
     if not (os.path.exists(obj) and os.path.exists(ref)):
         pytest.skip("shim objects not built")
     nm = lambda p: {l.split()[-1] for l in subprocess.run(["nm", "-g", "--defined-only", p], stdout=subprocess.PIPE, text=True).stdout.splitlines() if " T " in l}

@@ -37,7 +37,7 @@ def load(name):
 @pytest.fixture(scope="module")
 def dropin(gpu_lib):
     if not os.path.exists(DROPIN):
-        pytest.fail("tests/dropin/_build/libdsp_dropin.so missing (built by __graft_entry__.build() where /root/reference exists)")
+        pytest.fail("tests/dropin/_build/libdsp_dropin.so missing (linked by __graft_entry__.build() from the objects oracle/Makefile builds where the reference's sources are present)")
     from oracle import ref
     return ref
 

@@ -14,6 +14,12 @@ from conftest import rms
 
 pytestmark = pytest.mark.gpu
 RMS_TOL = 1e-10
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def ref_sample(name):
+    """Rows of the compiled reference's output on a test's own input (tests/golden/make_golden.py)."""
+    return np.load(os.path.join(GOLDEN, name + ".npz"))
 
 
 @contextmanager
@@ -90,6 +96,10 @@ def test_headline_composition_against_compiled_reference(gpu_lib, have_ref, tmp_
     assert got.shape == want.shape
     assert rms(got - want) <= RMS_TOL, (variant, rms(got - want))
     assert np.max(np.abs(got - want)) <= 1e-9
+    g = ref_sample("ref_headline")
+    assert got.shape[0] == g["frames"]
+    assert rms(got[g["rows"]] - g["y"]) <= RMS_TOL, (variant, rms(got[g["rows"]] - g["y"]))
+    assert np.max(np.abs(got[g["rows"]] - g["y"])) <= 1e-9
 
 
 @pytest.mark.parametrize("pipe", [1, 0])
@@ -223,6 +233,9 @@ def test_config3_64_channels_full_size(gpu_lib, have_ref, tmp_path):
         want = np.concatenate([r.run(x[i:i + F, :4]) for i in range(0, nblk * F, F)])
         r.close()
         assert rms(got[:, :4] - want) <= RMS_TOL, rms(got[:, :4] - want)
+    g = ref_sample("ref_config3")
+    assert got.shape[0] == g["frames"]
+    assert rms(got[g["rows"], :4] - g["y"]) <= RMS_TOL, rms(got[g["rows"], :4] - g["y"])
     for c in (5, 31, 32, 63):
         want = restate.fir_stream(x[:, c:c + 1], h[:, c:c + 1])
         assert rms(got[:, c:c + 1] - want) <= RMS_TOL, (c, rms(got[:, c:c + 1] - want))

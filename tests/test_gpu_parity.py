@@ -1,6 +1,8 @@
 """GPU tier: seeded inputs at sizes beyond the golden fixtures against the oracle (the compiled
 reference when it travelled, else the numpy restatement), plus size-independent properties at
 BASELINE.json's full sizes (impulse -> IR, linearity)."""
+import os
+
 import numpy as np
 import pytest
 
@@ -8,6 +10,12 @@ from conftest import rms
 
 pytestmark = pytest.mark.gpu
 RMS_TOL = 1e-10
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def ref_sample(name):
+    """Rows of the compiled reference's output on a test's own input (tests/golden/make_golden.py)."""
+    return np.load(os.path.join(GOLDEN, name + ".npz"))
 
 
 def eq_coefs(gpu_lib, fs, n_stages):
@@ -120,6 +128,9 @@ def test_resample_ratios(gpu_lib, have_ref, rates):
     got, counts = ch.process(x, 1024)
     assert counts == list(wcounts)
     assert rms(got - want) <= RMS_TOL, rms(got - want)
+    g, k = ref_sample("ref_resample_ratios"), "%d_%d_" % (fi, fo)
+    assert counts == list(g[k + "counts"])
+    assert rms(got[g[k + "rows"]] - g[k + "y"]) <= RMS_TOL
     ch.close()
 
 
@@ -139,7 +150,7 @@ def test_resample_channel_counts_pick_every_kernel_variant(gpu_lib, have_ref, ch
     else:
         r = restate.Resampler(fi, fo, channels)
     ch = gpu_lib.Chain(fi, channels).add_resample(fo)
-    pos = 0
+    pos, outs = 0, []
     for n in sizes:
         blk = x[pos:pos + n]
         pos += n
@@ -148,7 +159,11 @@ def test_resample_channel_counts_pick_every_kernel_variant(gpu_lib, have_ref, ch
         assert got.shape == want.shape
         if want.size:
             assert rms(got - want) <= RMS_TOL
+        outs.append(got)
     ch.close()
+    g, k = ref_sample("ref_resample_channels"), "%d_" % channels
+    assert [y.shape[0] for y in outs] == list(g[k + "counts"])
+    assert rms(np.concatenate(outs)[g[k + "rows"]][:, g[k + "cols"]] - g[k + "y"]) <= RMS_TOL
 
 
 def test_full_size_impulse_response_property(gpu_lib):
@@ -413,13 +428,18 @@ def test_full_size_config4_resample(gpu_lib, have_ref):
     else:
         r = restate.Resampler(fi, fo, 8)
     ch = gpu_lib.Chain(fi, C).add_resample(fo)
+    outs = []
     for i in range(0, nblk * F, F):
         want = r.run(base[i:i + F])
         got = ch.run(x[i:i + F]).copy()
         assert got.shape == (want.shape[0], C)
         assert rms(got[:, :8] - want) <= RMS_TOL
         assert np.array_equal(got, np.tile(got[:, :8], (1, C // 8)))
+        outs.append(got[:, :8])
     ch.close()
+    g = ref_sample("ref_config4")
+    assert [y.shape[0] for y in outs] == list(g["counts"])
+    assert rms(np.concatenate(outs)[g["rows"]] - g["y"]) <= RMS_TOL
 
 
 def test_full_size_config5_chain_share(gpu_lib, have_ref):

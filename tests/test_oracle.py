@@ -25,11 +25,9 @@ def test_golden_fixtures_present():
             "resample_2x", "chain"} <= set(names)
 
 
-def test_fftw_shim_against_numpy(have_ref):
-    if not have_ref:
-        pytest.skip("compiled reference not available")
-    from oracle import ref
-    L = ref.lib()
+def test_fftw_shim_against_numpy():
+    """oracle/fftw3_shim.c, the FFT backend of the compiled reference, built on its own by oracle/Makefile."""
+    L = C.CDLL(os.path.join(os.path.dirname(GOLDEN), "..", "oracle", "_ref", "libfftw3_shim.so"))
     L.fftw_plan_dft_r2c_1d.restype = C.c_void_p
     L.fftw_plan_dft_r2c_1d.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_uint]
     L.fftw_plan_dft_c2r_1d.restype = C.c_void_p
@@ -67,16 +65,16 @@ def test_compiled_reference_reproduces_golden(have_ref, name):
     assert np.array_equal(y, g["y"])
 
 
-def test_restated_sgen_matches_reference(have_ref):
-    if not have_ref:
-        pytest.skip("compiled reference not available")
-    from oracle import ref, restate
-    a = ref.sgen("sine+4800S", 48000, 2, 4800)
+def test_restated_sgen_matches_reference():
+    """Against the compiled reference's sgen output for the same specs (golden/ref_sgen.npz, make_golden.py)."""
+    from oracle import restate
+    g = load("ref_sgen")
+    a = g["tone"]                           # sgen "sine+4800S", 48 kHz, 2 channels
     b = restate.sgen_sine(48000, 2, 4800)
-    assert np.max(np.abs(a - b)) < 1e-12
-    a = ref.sgen("sine:freq=20-20k+4800S", 48000, 1, 4800)
+    assert a.shape == b.shape and np.max(np.abs(a - b)) < 1e-12
+    a = g["sweep"]                          # sgen "sine:freq=20-20k+4800S", 48 kHz, 1 channel
     b = restate.sgen_sine(48000, 1, 4800, 20.0, 20000.0)
-    assert np.max(np.abs(a - b)) < 1e-9
+    assert a.shape == b.shape and np.max(np.abs(a - b)) < 1e-9
 
 
 def test_restated_biquad_against_golden():
